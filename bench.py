@@ -17,6 +17,8 @@ Contract (see the task statement): `python bench.py --gpus N --steps K --warmup 
              with its own cpu_baseline (the oracle on one core over an SF1 database) at N=1
 `--impl reference` times the same reference code on all host cores, one process per core (the reference server itself cannot
 be built here: no bison/flex, see DESIGN.md), with the same metric / config keys; CBGPU_BENCH_CPU=port forces the restatement.
+`--dump-outputs DIR` also writes every query's result rows from its last timed step as DIR/<query>.npy; the inputs are generated
+from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -308,10 +310,25 @@ def traffic_of(kernel_name):
     return None
 
 
+def dump_outputs(path, results):
+    """--dump-outputs: each query's rows from its last timed step as DIR/<query>.npy, float64 of shape (rows, columns) in
+    the plan's output column order; numeric columns hold their decimal value, NULL is NaN.  The rows are sorted so that
+    two builds can be compared file by file whatever order their aggregates emit groups in."""
+    import math
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, rows in results.items():
+        vals = sorted(([float("nan") if x is None else float(x) for x in r] for r in rows),
+                      key=lambda r: [(math.isnan(x), 0.0 if math.isnan(x) else x) for x in r])
+        a = np.array(vals, dtype=np.float64).reshape(len(vals), len(vals[0]) if vals else 0)
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of every device-resident query (the end-to-end loop runs --e2e-steps)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--sf", type=float, default=100.0, help="scale factor of each GPU-segment's shard (default: the BASELINE config)")
@@ -323,7 +340,13 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=2)
     ap.add_argument("--no-joins", action="store_true", help="skip the Q3 / Q5 join pipelines (extra keys q3, q5)")
     ap.add_argument("--no-ssb", action="store_true", help="skip SSB Q4.1 - Q4.3 (extra key ssb)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write every query's result rows from its last timed step to DIR/<query>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path's rows; the reference arm has none")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -439,6 +462,7 @@ def main():
     clocks = sampler.stop()
     kname = knames[-1]
     q1_rows = bcast_rows(res.rows)
+    outputs = {"q1": q1_rows}        # --dump-outputs: each query's rows from its last timed step
     ngroups = len(q1_rows)
     ms = maxr([ms])[0]
     total_rows = nrows * world
@@ -591,7 +615,6 @@ def main():
     if not args.no_joins:
         from cloudberry_b200 import harness
         q5_sf = args.joins_sf if (args.joins_sf and world > 1) else (300.0 if (world == 8 and args.sf == 100.0) else args.sf)
-        jsteps = max(3, min(args.steps, 10))
         runs = [("q3", args.sf)] + [("q5", q5_sf)]
         if world > 1:
             ex.close()
@@ -617,10 +640,11 @@ def main():
             szj = tpch.sizes(int(jsf) if float(jsf).is_integer() else jsf)
             plan = (tpch.q3_plan(tpch.SEGMENTS.index("MACHINERY"), world, customer_replicated=False) if q == "q3"
                     else tpch.q5_plan(tpch.REGIONS.index("AMERICA"), world, replicated=False))
-            t = timed_query(exj, plan, jsteps)
+            t = timed_query(exj, plan, args.steps)
+            outputs[q] = t["rows"]
             rows_in, nbytes = harness.query_rows_bytes(q, szj)
             g = gold.get(BG.key(q, jsf))
-            joins[q] = {"value": rows_in / (t["ms"] / 1e3), "unit": "rows/s", "sf": jsf, "ms_per_step": t["ms"], "steps": jsteps, "rows_scanned": rows_in,
+            joins[q] = {"value": rows_in / (t["ms"] / 1e3), "unit": "rows/s", "sf": jsf, "ms_per_step": t["ms"], "steps": args.steps, "rows_scanned": rows_in,
                         "scaling": "strong" if world > 1 else "n/a", "result_rows": len(t["rows"]),
                         "result_check": result_check(q, t["rows"], (BG.q3_rows(g) if q == "q3" else BG.q5_rows(g)) if g else None,
                                                      "no golden rows for SF%g" % jsf),
@@ -650,16 +674,16 @@ def main():
         exs = capi.Executor(ctx, dev, motion=motion)
         rows_in, nbytes = ssb.query_rows_bytes(ssz)
         gs = gold.get(BG.key("ssb", args.sf))
-        ssteps = max(3, min(args.steps, 10))
         per, tot_ms = {}, 0.0
         for q in ("q4.1", "q4.2", "q4.3"):
-            t = timed_query(exs, ssb.PLANS[q](world), ssteps)
+            t = timed_query(exs, ssb.PLANS[q](world), args.steps)
+            outputs["ssb_" + q.replace(".", "_")] = t["rows"]
             tot_ms += t["ms"]
             per[q] = {"ms_per_step": t["ms"], "groups": len(t["rows"]), "longest_kernel": t["kernel"], "longest_kernel_ms": t["kernel_ms"],
                       "gpu_launches_per_step": t["launches"], "motion_bytes_per_step": t["sent"],
                       "result_check": result_check(q, t["rows"], BG.ssb_rows(gs, q) if gs else None, "no golden rows for SF%g" % args.sf),
                       "roofline_frac": nbytes / (t["ms"] / 1e3) / 1e9 / (peak * world)}
-        ssbres = {"value": 3 * rows_in / (tot_ms / 1e3), "unit": "rows/s", "sf": args.sf, "ms_per_step": tot_ms, "steps": ssteps,
+        ssbres = {"value": 3 * rows_in / (tot_ms / 1e3), "unit": "rows/s", "sf": args.sf, "ms_per_step": tot_ms, "steps": args.steps,
                   "rows_scanned": 3 * rows_in, "scaling": "strong" if world > 1 else "n/a", "queries": per,
                   "result_check": "ok" if all(v["result_check"] == "ok" for v in per.values()) else
                   next(v["result_check"] for v in per.values() if v["result_check"] != "ok"),
@@ -723,7 +747,9 @@ def main():
         line.update(joins)
         if ssbres:
             line["ssb"] = ssbres
-        print(json.dumps(line))
+        print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         if bad:
             sys.stderr.write("result_check FAILED: %s\n" % bad[0])
     if ex:

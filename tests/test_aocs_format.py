@@ -17,11 +17,13 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 def golden():
-    d = np.load(os.path.join(HERE, "golden", "aocs_columns.npz"))
-    for c in d["cases"]:
-        name, typname, checksum, blocksize, dscale, nblocks = str(c).split("|")
-        yield (name, typname, int(checksum), int(blocksize), int(dscale), int(nblocks), bytes(d[name + "__raw"]),
-               d[name + "__values"], d[name + "__nulls"])
+    """the uncompressed columns, split over two files to keep each under 1 MB"""
+    for f in ("aocs_columns.npz", "aocs_columns_2.npz"):
+        d = np.load(os.path.join(HERE, "golden", f))
+        for c in d["cases"]:
+            name, typname, checksum, blocksize, dscale, nblocks = str(c).split("|")
+            yield (name, typname, int(checksum), int(blocksize), int(dscale), int(nblocks), bytes(d[name + "__raw"]),
+                   d[name + "__values"], d[name + "__nulls"])
 
 
 CASES = list(golden())

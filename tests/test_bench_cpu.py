@@ -36,6 +36,18 @@ def test_reference_arm_line(force_port):
     assert line["e2e"] == {"value": line["value"], "unit": "rows/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_dump_outputs(tmp_path):
+    """result rows -> DIR/<query>.npy: float64, rows sorted, numeric text as its value, NULL as NaN (sorted last)"""
+    import bench
+    import numpy as np
+    bench.dump_outputs(str(tmp_path), {"q1": [[82, 70, "3774200.00", None], [65, 70, "-0.05", 7], [65, 70, "-0.05", None]],
+                                       "empty": []})
+    q1 = np.load(tmp_path / "q1.npy")
+    assert q1.dtype == np.float64
+    np.testing.assert_array_equal(q1, [[65, 70, -0.05, 7], [65, 70, -0.05, np.nan], [82, 70, 3774200.0, np.nan]])
+    assert np.load(tmp_path / "empty.npy").shape == (0, 0)
+
+
 def test_join_cpu_samples():
     import bench
     out = bench.cpu_join_samples(sf=0.1)

@@ -319,10 +319,15 @@ def gpu():
             "cbgpu_rel_col_devptr": (vp, [vp, i32]),
             "cbgpu_rel_nbytes": (C.c_size_t, [vp]),
             "cbgpu_ht_build": (C.c_int, [vp, vp, C.POINTER(i32), i32, C.POINTER(vp)]),
+            "cbgpu_ht_build_batched": (C.c_int, [vp, vp, C.POINTER(i32), i32, i32, C.POINTER(vp)]),
+            "cbgpu_ht_nbatch": (C.c_int, [vp]),
+            "cbgpu_ht_bytes_for": (i64, [i64]),
             "cbgpu_ht_free": (None, [vp]),
             "cbgpu_ht_nrows": (i64, [vp]),
             "cbgpu_ht_has_duplicates": (C.c_int, [vp]),
             "cbgpu_ht_probe_pairs": (C.c_int, [vp, vp, vp, C.POINTER(i32), i32, vp, i64, vp]),
+            # pending: a PENDING_FN or None
+            "cbgpu_ht_probe_pairs_batched": (C.c_int, [vp, vp, vp, C.POINTER(i32), i32, i32, i32, vp, vp, C.POINTER(i64), vp]),
             "cbgpu_pairs_free": (None, [vp]),
             "cbgpu_merge_sorted_runs": (C.c_int, [vp, vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), i32, i32, C.POINTER(vp),
                                                   C.POINTER(i32)]),
@@ -500,6 +505,12 @@ class Context:
 
 
 ALLGATHER_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t)
+PENDING_FN = C.CFUNCTYPE(C.c_int, C.c_void_p)
+
+
+class CbgpuPairs(C.Structure):
+    """cbgpu_pairs: npairs (outer_idx, inner_idx) row-id pairs in two device arrays; 0xFFFFFFFF = the side is missing"""
+    _fields_ = [("npairs", C.c_int64), ("outer_idx", C.c_void_p), ("inner_idx", C.c_void_p)]
 
 
 class Motion:
@@ -831,7 +842,7 @@ class Executor:
 class Cluster:
     """N segment executors in one process over one GPU (the reference's gpdemo, on a device)."""
 
-    def __init__(self, ctx, segment_range_tables, force_generic=False):
+    def __init__(self, ctx, segment_range_tables, force_generic=False, operator_mem_kb=0):
         self.ctx = ctx
         self.E = ex()
         self.nsegs = len(segment_range_tables)
@@ -844,6 +855,7 @@ class Cluster:
             if rc:
                 raise CbgpuError(rc, "bad range table")
             self.E.cb_cluster_estate(self.h, s).contents.es_force_generic = 1 if force_generic else 0
+            self.E.cb_cluster_estate(self.h, s).contents.es_operator_mem_kb = int(operator_mem_kb)
 
     def run(self, plan_node):
         E = self.E

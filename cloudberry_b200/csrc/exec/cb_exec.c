@@ -614,6 +614,15 @@ stream_over_rel(CbEState *es, CbStream *s, cbgpu_rel *rel, const PExpr *shape, i
 	return CBGPU_OK;
 }
 
+/* the caller's interrupt check in the form the device library polls between hash join batches */
+static int
+es_pending(void *arg)
+{
+	CbEState   *es = (CbEState *) arg;
+
+	return es->es_interrupt_pending && es->es_interrupt_pending(es);
+}
+
 /*
  * Run a pipeline.  When one of its probes is a multi-batch hash join (the build side did not fit the operator's memory,
  * nodeHash.c:980-990) the pipeline runs once per batch, each pass with that batch of the build side resident and the
@@ -1058,8 +1067,21 @@ open_hashjoin(CbPlanState *ps, CbStream **out)
 		NodePriv   *me = np(ps);
 		int			c;
 
-		if (cbgpu_ht_nbatch(hp->ht) > 1)
-			return es_fail(es, CBGPU_ERR_UNSUPPORTED, "multi-batch hash join with duplicate build keys is not implemented on the GPU path (raise the operator memory)");
+		const int	multi = cbgpu_ht_nbatch(hp->ht) > 1;
+
+		if (multi)
+			/* the batched probe loads build batches by key hash: the same key checks as the pipelined probe below */
+			for (int k = 0; k < hj->nhashkeys; k++)
+			{
+				PExpr	   *kx = &s->pe[keys[k]];
+
+				if (kx->type == CB_FLOAT8)
+					return es_fail(es, CBGPU_ERR_UNSUPPORTED, "float8 join keys are not on the GPU path");
+				if ((kx->type == CB_DICT8 || kx->type == CB_DICT32) &&
+					(kx->kind != PE_COL || !s->pipe.cols[kx->col].dict_hash ||
+					 cbgpu_ht_key_dict_hash(hp->ht, k) != s->pipe.cols[kx->col].dict_hash))
+					return es_fail(es, CBGPU_ERR_UNSUPPORTED, "join of dictionary columns coded by two different dictionaries (share one dictionary between the columns)");
+			}
 		/* append the key expressions as extra output columns so the probe can read them */
 		for (int k = 0; k < hj->nhashkeys; k++)
 		{
@@ -1076,7 +1098,18 @@ open_hashjoin(CbPlanState *ps, CbStream **out)
 		if (me->owned.npairs >= 8)
 			return es_fail(es, CBGPU_ERR_UNSUPPORTED, "too many N:M joins under one node");
 		pairs = &me->owned.pairs[me->owned.npairs++];
-		GPU(es, cbgpu_ht_probe_pairs_outer(es->es_ctx, hp->ht, orel, keycols, hj->nhashkeys, fill_outer, fill_inner, pairs));
+		if (multi)
+		{
+			/* build side split into batches: the probe rows are grouped by batch once, each batch is loaded and probed in
+			 * turn (HJ_NEED_NEW_BATCH, nodeHashjoin.c:709-738), unmatched build rows follow the last batch */
+			int64_t		passes = 0;
+
+			GPU(es, cbgpu_ht_probe_pairs_batched(es->es_ctx, hp->ht, orel, keycols, hj->nhashkeys, fill_outer,
+												 fill_inner, es_pending, es, &passes, pairs));
+			es->es_hashjoin_batches_run += passes;
+		}
+		else
+			GPU(es, cbgpu_ht_probe_pairs_outer(es->es_ctx, hp->ht, orel, keycols, hj->nhashkeys, fill_outer, fill_inner, pairs));
 		s2 = stream_new(me);
 		TRY(stream_over_rel(es, s2, orel, shape, nouter));
 		if (fill_inner)

@@ -444,6 +444,10 @@ struct ProbeParams
 	const uint32_t *sel;
 	int64_t		n;
 	int32_t		left;			/* LEFT join: an outer row without a partner yields one pair (row, 0xFFFFFFFF)  */
+	int32_t		presel;			/* every row of sel belongs to the resident batch (k_ht_partition_*): an unmatched
+								 * LEFT row is emitted whatever its key hash - a NULL key's hash is not its batch */
+	int32_t		sort_matches;	/* the build side has duplicate keys: a row's partners are written in build row order,
+								 * not in the order the table's fill happened to place them */
 	uint8_t    *matched;		/* RIGHT / FULL join: [inner rows] set to 1 for every build row that found a partner
 								 * (HeapTupleHeaderSetMatch, nodeHashjoin.c:560); NULL otherwise */
 	int64_t		ninner;
@@ -451,6 +455,66 @@ struct ProbeParams
 	uint32_t   *out_outer;
 	uint32_t   *out_inner;
 };
+
+struct KeyHash
+{
+	uint32_t	h;
+	bool		isnull;			/* some key is NULL: h is not the row's hash (the reference's keep_nulls hash is 0) */
+};
+
+/* a probe row's key hash (and its key values, into key[]): the pair probe and the partition of the probe side by batch
+ * both hash through here, so a row is probed in the pass of the batch it was filed under */
+__device__ __forceinline__ KeyHash
+pp_key_hash(const ProbeParams &p, uint32_t row, int64_t *key)
+{
+	KeyHash		r = {0, false};
+
+	for (int k = 0; k < p.ht.nkeys; k++)
+	{
+		if (p.onulls[k] && p.onulls[k][row])
+			r.isnull = true;
+		key[k] = cb_load_widen(p.okey[k], p.otype[k], row);
+		r.h = pg_hash_combine(r.h, jh_hash_datum(p.otype[k], key[k], p.odict[k]), false);
+	}
+	return r;
+}
+
+/* heapsort of a short run of row ids, in place: deterministic whatever the input, O(n log n) however many duplicates */
+__device__ __forceinline__ void
+u32_sift_down(uint32_t *a, int64_t root, int64_t end)
+{
+	uint32_t	v = a[root];
+
+	for (;;)
+	{
+		int64_t		c = 2 * root + 1;
+
+		if (c >= end)
+			break;
+		if (c + 1 < end && a[c + 1] > a[c])
+			c++;
+		if (a[c] <= v)
+			break;
+		a[root] = a[c];
+		root = c;
+	}
+	a[root] = v;
+}
+
+__device__ void
+u32_sort(uint32_t *a, int64_t n)
+{
+	for (int64_t i = n / 2; i-- > 0;)
+		u32_sift_down(a, i, n);
+	for (int64_t e = n - 1; e > 0; e--)
+	{
+		uint32_t	t = a[0];
+
+		a[0] = a[e];
+		a[e] = t;
+		u32_sift_down(a, 0, e);
+	}
+}
 
 template <bool WRITE>
 __global__ void __launch_bounds__(256)
@@ -462,19 +526,13 @@ k_ht_probe_pairs(ProbeParams p)
 	for (; i < p.n; i += stride)
 	{
 		uint32_t	row = p.sel ? p.sel[i] : (uint32_t) i;
-		uint32_t	h = 0;
 		int64_t		key[CBP_MAX_KEYS];
-		bool		isnull = false;
+		const KeyHash kh = pp_key_hash(p, row, key);
+		const uint32_t h = kh.h;
+		bool		isnull = kh.isnull;
 		unsigned long long cnt = 0;
 		unsigned long long base = WRITE ? p.counts[i] : 0;
 
-		for (int k = 0; k < p.ht.nkeys; k++)
-		{
-			if (p.onulls[k] && p.onulls[k][row])
-				isnull = true;
-			key[k] = cb_load_widen(p.okey[k], p.otype[k], row);
-			h = pg_hash_combine(h, jh_hash_datum(p.otype[k], key[k], p.odict[k]), false);
-		}
 		if (!isnull && p.ht.bloom)
 		{
 			uint32_t	w;
@@ -520,7 +578,9 @@ k_ht_probe_pairs(ProbeParams p)
 				pos = (pos + 1) & p.ht.mask;
 			}
 		}
-		if (p.left && cnt == 0 && ht_in_batch(p.ht.nbatch, p.ht.batch_shift, p.ht.batch_id, h))
+		if (WRITE && p.sort_matches && cnt > 1)
+			u32_sort(p.out_inner + base, (int64_t) cnt);	/* this thread's own run of pairs: one outer row */
+		if (p.left && cnt == 0 && (p.presel || ht_in_batch(p.ht.nbatch, p.ht.batch_shift, p.ht.batch_id, h)))
 		{
 			/* no partner (or a NULL key, which never has one): the outer row survives with a NULL inner side */
 			if (WRITE)
@@ -621,6 +681,144 @@ k_ht_unmatched_write(ProbeParams p)
 		}
 }
 
+/* ---------------------------------------------------------------------------------------------
+ * The probe side grouped by hash-join batch (the reference writes outer tuples to per-batch temp files, ExecHashJoinSaveTuple
+ * nodeHashjoin.c:1060; here the row ids are grouped once in HBM): ids[off[b] .. off[b+1]) are the rows of batch b, in row
+ * order.  A NULL-keyed row belongs to batch 0, as in the pipelined probe (pipeline.cu, keep_nulls hash 0).  Two passes over
+ * the key columns: per-CTA histograms (each CTA owns one contiguous range of rows) into a batch-major [nbatch][nCTA] matrix,
+ * its exclusive scan, then an in-order scatter of each range.
+ * --------------------------------------------------------------------------------------------- */
+#define PART_THREADS 256
+
+__device__ __forceinline__ uint32_t
+pp_row_batch(const ProbeParams &p, uint32_t row, int32_t batch_shift)
+{
+	int64_t		key[CBP_MAX_KEYS];
+	const KeyHash kh = pp_key_hash(p, row, key);
+
+	return kh.isnull ? 0 : kh.h >> batch_shift;
+}
+
+__global__ void __launch_bounds__(PART_THREADS)
+k_ht_partition_count(ProbeParams p, int32_t nbatch, int32_t batch_shift, int64_t chunk, unsigned long long *counts)
+{
+	extern __shared__ uint32_t s_hist[];
+	const int64_t lo = (int64_t) blockIdx.x * chunk;
+	const int64_t hi = lo + chunk < p.n ? lo + chunk : p.n;
+
+	for (int b = threadIdx.x; b < nbatch; b += blockDim.x)
+		s_hist[b] = 0;
+	__syncthreads();
+	for (int64_t t = lo; t < hi; t += blockDim.x)
+	{
+		const int64_t i = t + threadIdx.x;
+		const uint32_t b = i < hi ? pp_row_batch(p, (uint32_t) i, batch_shift) : 0xFFFFFFFFu;
+		const unsigned peers = __match_any_sync(0xffffffffu, b);
+
+		/* one shared atomic per batch present in the warp (few batches: every lane would hit the same word) */
+		if (b != 0xFFFFFFFFu && (threadIdx.x & 31) == __ffs(peers) - 1)
+			atomicAdd(&s_hist[b], (uint32_t) __popc(peers));
+	}
+	__syncthreads();
+	for (int b = threadIdx.x; b < nbatch; b += blockDim.x)
+		counts[(int64_t) b * gridDim.x + blockIdx.x] = s_hist[b];
+}
+
+__global__ void __launch_bounds__(PART_THREADS)
+k_ht_partition_scatter(ProbeParams p, int32_t nbatch, int32_t batch_shift, int64_t chunk, const unsigned long long *scan,
+					   uint32_t *ids, unsigned long long *off)
+{
+	extern __shared__ uint32_t s_next[];	/* where this CTA's next row of each batch goes */
+	const int64_t lo = (int64_t) blockIdx.x * chunk;
+	const int64_t hi = lo + chunk < p.n ? lo + chunk : p.n;
+	const int	lane = threadIdx.x & 31,
+				warp = threadIdx.x >> 5;
+
+	for (int b = threadIdx.x; b < nbatch; b += blockDim.x)
+	{
+		s_next[b] = (uint32_t) scan[(int64_t) b * gridDim.x + blockIdx.x];
+		if (blockIdx.x == 0)
+			off[b] = scan[(int64_t) b * gridDim.x];
+	}
+	if (blockIdx.x == 0 && threadIdx.x == 0)
+		off[nbatch] = scan[(int64_t) nbatch * gridDim.x];
+	__syncthreads();
+	for (int64_t t = lo; t < hi; t += blockDim.x)
+	{
+		const int64_t i = t + threadIdx.x;
+		const bool	v = i < hi;
+		const uint32_t b = v ? pp_row_batch(p, (uint32_t) i, batch_shift) : 0xFFFFFFFFu;
+		const unsigned peers = __match_any_sync(0xffffffffu, b);
+		const int	rank = __popc(peers & ((1u << lane) - 1));
+
+		/* the warps of the tile take their places in order, so every batch's ids stay in row order */
+		for (int w = 0; w < PART_THREADS / 32; w++)
+		{
+			uint32_t	at = 0;
+
+			if (w == warp && v)
+				at = s_next[b];
+			__syncwarp();
+			if (w == warp && v)
+			{
+				ids[at + rank] = (uint32_t) i;
+				if (lane == __ffs(peers) - 1)
+					s_next[b] = at + __popc(peers);
+			}
+			__syncthreads();
+		}
+	}
+}
+
+#define HT_TRY(call) \
+	do { \
+		int rc__ = (call); \
+		if (rc__ != CBGPU_OK) \
+			return rc__; \
+	} while (0)
+
+/* device scratch of one batched pair probe, freed whatever the outcome */
+struct PairsBatchedScratch
+{
+	unsigned long long *part;	/* [nbatch * nCTA + 1] histogram matrix, then its scan                */
+	unsigned long long *off;	/* [nbatch + 1] batch offsets into ids                                */
+	uint32_t   *ids;			/* [outer rows] grouped by batch                                     */
+	unsigned long long *counts;	/* [max(rows of a batch, inner rows) + 1]                             */
+	uint8_t    *matched;		/* [inner rows] RIGHT / FULL                                          */
+	unsigned long long *h_off;	/* host copy of off                                                   */
+};
+
+/* p.n probe rows (no selection) -> s->ids grouped by batch, h_off[nbatch + 1] their offsets (one read-back) */
+static int
+ht_partition_probe(cbgpu_ctx *ctx, const ProbeParams &p, int32_t nbatch, int32_t batch_shift, PairsBatchedScratch *s,
+				   unsigned long long *h_off)
+{
+	const int64_t cap = 262144;	/* matrix entries: its single-CTA scan stays well under a millisecond */
+	int64_t		g = (p.n + 8 * PART_THREADS - 1) / (8 * PART_THREADS);
+
+	if (g > 2 * (int64_t) ctx->sm_count)
+		g = 2 * (int64_t) ctx->sm_count;
+	if (g > cap / nbatch)
+		g = cap / nbatch;
+	if (g < 1)
+		g = 1;
+	const int64_t chunk = (p.n + g - 1) / g;
+	const size_t shmem = sizeof(uint32_t) * (size_t) nbatch;	/* <= 16 KB */
+
+	CB_CUDA(ctx, cudaMallocAsync(&s->part, sizeof(unsigned long long) * (size_t) (nbatch * g + 1), ctx->stream));
+	CB_CUDA(ctx, cudaMallocAsync(&s->off, sizeof(unsigned long long) * (size_t) (nbatch + 1), ctx->stream));
+	CB_CUDA(ctx, cudaMallocAsync(&s->ids, sizeof(uint32_t) * (size_t) p.n, ctx->stream));
+	k_ht_partition_count<<<(unsigned) g, PART_THREADS, shmem, ctx->stream>>>(p, nbatch, batch_shift, chunk, s->part);
+	CB_LAUNCHED(ctx, "k_ht_partition_count");
+	k_exclusive_scan_u64<<<1, 1024, 0, ctx->stream>>>(s->part, nbatch * g);
+	CB_LAUNCHED(ctx, "k_exclusive_scan_u64");
+	k_ht_partition_scatter<<<(unsigned) g, PART_THREADS, shmem, ctx->stream>>>(p, nbatch, batch_shift, chunk, s->part, s->ids, s->off);
+	CB_LAUNCHED(ctx, "k_ht_partition_scatter");
+	CB_CUDA(ctx, cudaMemcpyAsync(h_off, s->off, sizeof(unsigned long long) * (size_t) (nbatch + 1), cudaMemcpyDeviceToHost, ctx->stream));
+	CB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+	return CBGPU_OK;
+}
+
 static int	ht_probe_pairs(cbgpu_ctx *ctx, const cbgpu_hashtable *ht, cbgpu_rel *outer, const int32_t *keycols, int32_t nkeys,
 						   const uint32_t *sel, int64_t nsel, int left, int fill_inner, cbgpu_pairs *out);
 
@@ -645,6 +843,203 @@ cbgpu_ht_probe_pairs_left(cbgpu_ctx *ctx, const cbgpu_hashtable *ht, cbgpu_rel *
 	return ht_probe_pairs(ctx, ht, outer, keycols, nkeys, NULL, 0, 1, 0, out);
 }
 
+/* the probe side's key columns into a zeroed ProbeParams over the table as it is now */
+static int
+pp_setup(cbgpu_ctx *ctx, const cbgpu_hashtable *ht, cbgpu_rel *outer, const int32_t *keycols, int32_t nkeys, ProbeParams *p)
+{
+	if (nkeys != ht->d.nkeys)
+		return cb_fail(ctx, CBGPU_ERR_INVALID, "cbgpu_ht_probe_pairs: key count mismatch%s %lld", "", nkeys);
+	memset(p, 0, sizeof(*p));
+	p->ht = ht->d;
+	for (int k = 0; k < nkeys; k++)
+	{
+		int			c = keycols[k];
+
+		if (c < 0 || c >= outer->ncols)
+			return cb_fail(ctx, CBGPU_ERR_INVALID, "cbgpu_ht_probe_pairs: bad key column%s %lld", "", c);
+		p->okey[k] = outer->data[c];
+		p->onulls[k] = outer->nulls[c];
+		p->odict[k] = outer->dict_hash[c];
+		p->otype[k] = outer->types[c];
+	}
+	return CBGPU_OK;
+}
+
+/* room for `need` pairs in out's arrays (cudaMalloc'd: cbgpu_pairs_free frees them), growing geometrically */
+static int
+pairs_reserve(cbgpu_ctx *ctx, cbgpu_pairs *out, int64_t *cap, int64_t need)
+{
+	uint32_t   *o,
+			   *in;
+	int64_t		ncap = *cap * 2 > need ? *cap * 2 : need;
+	cudaError_t e;
+
+	if (need <= *cap)
+		return CBGPU_OK;
+	if (ncap > 0xFFFFFFF0ll)
+		ncap = 0xFFFFFFF0ll;
+	CB_CUDA(ctx, cudaMalloc(&o, (size_t) ncap * sizeof(uint32_t)));
+	if ((e = cudaMalloc(&in, (size_t) ncap * sizeof(uint32_t))) != cudaSuccess)
+		cudaFree(o);
+	CB_CUDA(ctx, e);
+	if (out->npairs)
+	{
+		CB_CUDA(ctx, cudaMemcpyAsync(o, out->outer_idx, (size_t) out->npairs * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+		CB_CUDA(ctx, cudaMemcpyAsync(in, out->inner_idx, (size_t) out->npairs * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+		CB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+	}
+	if (out->outer_idx)
+		cudaFree(out->outer_idx);
+	if (out->inner_idx)
+		cudaFree(out->inner_idx);
+	out->outer_idx = o;
+	out->inner_idx = in;
+	*cap = ncap;
+	return CBGPU_OK;
+}
+
+/* p.counts[0 .. p.n) just counted: scan them, make room and append the pairs the write kernel `write` emits */
+template <typename W>
+static int
+pairs_append(cbgpu_ctx *ctx, ProbeParams &p, int64_t nitems, cbgpu_pairs *out, int64_t *cap, W write)
+{
+	unsigned long long total = 0;
+
+	k_exclusive_scan_u64<<<1, 1024, 0, ctx->stream>>>(p.counts, nitems);
+	CB_LAUNCHED(ctx, "k_exclusive_scan_u64");
+	CB_CUDA(ctx, cudaMemcpyAsync(&total, p.counts + nitems, sizeof(total), cudaMemcpyDeviceToHost, ctx->stream));
+	CB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+	if (total + (unsigned long long) out->npairs > 0xFFFFFFF0ull)
+		return cb_fail(ctx, CBGPU_ERR_UNSUPPORTED, "join result of %s%lld pairs exceeds the GPU path's 32-bit row ids", "",
+					   (long long) (total + (unsigned long long) out->npairs));
+	if (total == 0)
+		return CBGPU_OK;
+	HT_TRY(pairs_reserve(ctx, out, cap, out->npairs + (int64_t) total));
+	p.out_outer = out->outer_idx + out->npairs;
+	p.out_inner = out->inner_idx + out->npairs;
+	HT_TRY(write());
+	out->npairs += (int64_t) total;
+	return CBGPU_OK;
+}
+
+static int
+ht_probe_pairs_batched(cbgpu_ctx *ctx, cbgpu_hashtable *ht, cbgpu_rel *outer, const int32_t *keycols, int32_t nkeys, int left,
+					   int fill_inner, int (*pending)(void *), void *pending_arg, int64_t *passes, PairsBatchedScratch *s,
+					   cbgpu_pairs *out)
+{
+	ProbeParams p;
+	const int32_t nbatch = ht->d.nbatch;
+	const int64_t n = outer->nrows;
+	const int64_t ninner = fill_inner ? ht->inner->nrows : 0;
+	int64_t		maxrows = ninner,
+				cap = 0;
+
+	HT_TRY(pp_setup(ctx, ht, outer, keycols, nkeys, &p));
+	if (n + ninner == 0)
+		return CBGPU_OK;
+	s->h_off = (unsigned long long *) calloc((size_t) nbatch + 1, sizeof(unsigned long long));
+	if (!s->h_off)
+		return CBGPU_ERR_NOMEM;
+	if (n > 0)
+	{
+		p.n = n;
+		HT_TRY(ht_partition_probe(ctx, p, nbatch, ht->d.batch_shift, s, s->h_off));
+	}
+	for (int b = 0; b < nbatch; b++)
+		if ((int64_t) (s->h_off[b + 1] - s->h_off[b]) > maxrows)
+			maxrows = (int64_t) (s->h_off[b + 1] - s->h_off[b]);
+	CB_CUDA(ctx, cudaMallocAsync(&s->counts, (size_t) (maxrows + 1) * sizeof(unsigned long long), ctx->stream));
+	if (ninner)
+	{
+		CB_CUDA(ctx, cudaMallocAsync(&s->matched, (size_t) ninner, ctx->stream));
+		CB_CUDA(ctx, cudaMemsetAsync(s->matched, 0, (size_t) ninner, ctx->stream));
+	}
+	p.counts = s->counts;
+	p.matched = s->matched;
+	p.left = left;
+	p.presel = 1;
+	p.sort_matches = ht->has_dups;
+	for (int b = 0; b < nbatch; b++)
+	{
+		const int64_t lo = (int64_t) s->h_off[b];
+		const int64_t cnt = (int64_t) (s->h_off[b + 1] - s->h_off[b]);
+
+		if (cnt <= 0 || lo < 0 || lo + cnt > n)
+			continue;			/* no probe row in this batch: its build rows need no table (the unmatched pass reads matched) */
+		/* HJ_NEED_NEW_BATCH (nodeHashjoin.c:709): the caller's CHECK_FOR_INTERRUPTS between batches */
+		if (pending && pending(pending_arg))
+			return cb_fail(ctx, CBGPU_ERR_INTERRUPTED, "canceling statement due to user request%s", "");
+		HT_TRY(cbgpu_ht_load_batch(ht, b));
+		p.ht = ht->d;
+		p.sel = s->ids + lo;
+		p.n = cnt;
+
+		const int	blocks = (int) ((cnt + 255) / 256 < ctx->sm_count * 8 ? (cnt + 255) / 256 : ctx->sm_count * 8);
+
+		k_ht_probe_pairs<false><<<blocks, 256, 0, ctx->stream>>>(p);
+		CB_LAUNCHED(ctx, "k_ht_probe_pairs<count>");
+		HT_TRY(pairs_append(ctx, p, cnt, out, &cap, [&]() {
+			k_ht_probe_pairs<true><<<blocks, 256, 0, ctx->stream>>>(p);
+			CB_LAUNCHED(ctx, "k_ht_probe_pairs<write>");
+			return CBGPU_OK;
+		}));
+		(*passes)++;
+	}
+	if (ninner)
+	{
+		/* HJ_FILL_INNER_TUPLES once, after the last batch: build rows of every batch that no probe row matched, NULL-keyed
+		 * ones (never inserted in any batch) included */
+		const int	iblocks = (int) ((ninner + 255) / 256 < ctx->sm_count * 8 ? (ninner + 255) / 256 : ctx->sm_count * 8);
+
+		p.sel = NULL;
+		p.n = 0;
+		p.ninner = ninner;
+		k_ht_unmatched_count<<<iblocks, 256, 0, ctx->stream>>>(p);
+		CB_LAUNCHED(ctx, "k_ht_unmatched_count");
+		HT_TRY(pairs_append(ctx, p, ninner, out, &cap, [&]() {
+			k_ht_unmatched_write<<<iblocks, 256, 0, ctx->stream>>>(p);
+			CB_LAUNCHED(ctx, "k_ht_unmatched_write");
+			return CBGPU_OK;
+		}));
+	}
+	return CBGPU_OK;
+}
+
+extern "C" int
+cbgpu_ht_probe_pairs_batched(cbgpu_ctx *ctx, cbgpu_hashtable *ht, cbgpu_rel *outer, const int32_t *keycols, int32_t nkeys,
+							 int32_t fill_outer, int32_t fill_inner, int (*pending)(void *), void *pending_arg, int64_t *passes,
+							 cbgpu_pairs *out)
+{
+	PairsBatchedScratch s;
+	int			rc;
+
+	*passes = 0;
+	if (ht->d.nbatch <= 1)
+	{
+		rc = ht_probe_pairs(ctx, ht, outer, keycols, nkeys, NULL, 0, fill_outer != 0, fill_inner != 0, out);
+		*passes = rc == CBGPU_OK && outer->nrows > 0;
+		return rc;
+	}
+	memset(out, 0, sizeof(*out));
+	memset(&s, 0, sizeof(s));
+	rc = ht_probe_pairs_batched(ctx, ht, outer, keycols, nkeys, fill_outer != 0, fill_inner != 0, pending, pending_arg, passes, &s, out);
+	cudaSetDevice(ctx->device);
+	if (s.part)
+		cudaFreeAsync(s.part, ctx->stream);
+	if (s.off)
+		cudaFreeAsync(s.off, ctx->stream);
+	if (s.ids)
+		cudaFreeAsync(s.ids, ctx->stream);
+	if (s.counts)
+		cudaFreeAsync(s.counts, ctx->stream);
+	if (s.matched)
+		cudaFreeAsync(s.matched, ctx->stream);
+	free(s.h_off);
+	if (rc != CBGPU_OK)
+		cbgpu_pairs_free(out);
+	return rc;
+}
+
 static int
 ht_probe_pairs(cbgpu_ctx *ctx, const cbgpu_hashtable *ht, cbgpu_rel *outer, const int32_t *keycols, int32_t nkeys,
 			   const uint32_t *sel, int64_t nsel, int left, int fill_inner, cbgpu_pairs *out)
@@ -655,21 +1050,7 @@ ht_probe_pairs(cbgpu_ctx *ctx, const cbgpu_hashtable *ht, cbgpu_rel *outer, cons
 	const int64_t ninner = fill_inner ? ht->inner->nrows : 0;
 
 	memset(out, 0, sizeof(*out));
-	if (nkeys != ht->d.nkeys)
-		return cb_fail(ctx, CBGPU_ERR_INVALID, "cbgpu_ht_probe_pairs: key count mismatch%s %lld", "", nkeys);
-	memset(&p, 0, sizeof(p));
-	p.ht = ht->d;
-	for (int k = 0; k < nkeys; k++)
-	{
-		int			c = keycols[k];
-
-		if (c < 0 || c >= outer->ncols)
-			return cb_fail(ctx, CBGPU_ERR_INVALID, "cbgpu_ht_probe_pairs: bad key column%s %lld", "", c);
-		p.okey[k] = outer->data[c];
-		p.onulls[k] = outer->nulls[c];
-		p.odict[k] = outer->dict_hash[c];
-		p.otype[k] = outer->types[c];
-	}
+	HT_TRY(pp_setup(ctx, ht, outer, keycols, nkeys, &p));
 	p.sel = sel;
 	p.n = n;
 	p.left = left;

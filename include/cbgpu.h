@@ -324,6 +324,15 @@ int			cbgpu_ht_probe_pairs_left(cbgpu_ctx *ctx, const cbgpu_hashtable *ht, cbgpu
  * FULL: ExecScanHashTableForUnmatched nodeHash.c:2360, HJ_FILL_INNER_TUPLES nodeHashjoin.c:676-706) */
 int			cbgpu_ht_probe_pairs_outer(cbgpu_ctx *ctx, const cbgpu_hashtable *ht, cbgpu_rel *outer, const int32_t *keycols,
 									   int32_t nkeys, int32_t fill_outer, int32_t fill_inner, cbgpu_pairs *out);
+/* every outer-join flavour of the pair probe (as cbgpu_ht_probe_pairs_outer) over a table of any batch count: the probe rows
+ * are grouped by batch once (a NULL-keyed row in batch 0), each batch with probe rows is loaded and probed in turn, and the
+ * build rows no probe row matched are emitted once after the last batch.  Pairs come in (batch, outer row) order - a row's
+ * partners in build row order - then the unmatched build rows in row order.  pending(pending_arg), when given, is polled
+ * before each batch (nonzero: CBGPU_ERR_INTERRUPTED); *passes = batches probed.  The table is left on the last batch the
+ * call loaded (a single-batch table: the cbgpu_ht_probe_pairs_outer path, unchanged). */
+int			cbgpu_ht_probe_pairs_batched(cbgpu_ctx *ctx, cbgpu_hashtable *ht, cbgpu_rel *outer, const int32_t *keycols,
+										 int32_t nkeys, int32_t fill_outer, int32_t fill_inner, int (*pending) (void *),
+										 void *pending_arg, int64_t *passes, cbgpu_pairs *out);
 void		cbgpu_pairs_free(cbgpu_pairs *p);
 int			cbgpu_read_u32(cbgpu_ctx *ctx, const uint32_t *dev, int64_t n, uint32_t *host);
 /* small device scratch (sink row counters, index vectors): zero-filled allocation, read-back, free */
